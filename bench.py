@@ -5,6 +5,7 @@
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA path through the public API)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU implementation of the path
     python bench.py --workload C1|C2|C3|C4                   # other BASELINE.json configs (default C3, the metric's)
+    python bench.py --dump-outputs DIR ...                   # also write the outputs of the last timed step (DIR/*.npy)
 
 A "step" is one pass of the hot path over one BATCH of synthetic views: `--views-per-step` (default 32) fused
 deform + rasterize FORWARDS of the workload, back to back -- so that `--steps 20` times >= 0.5 s of device work instead of
@@ -276,14 +277,21 @@ def run_ours(args):
         torch.cuda.synchronize(dev)
 
     # ------------------------------------------------------------------ resident arm (`value`)
-    def resident_step(step):
+    def resident_step(step, kept=None):
         out = None
+        if kept is not None:
+            kept.clear()      # the previous step's outputs go back to the allocator before this step allocates its own
         for v in range(V):
             if v == V - 1:
                 ws.set_option(lib.OPT_STAGE_TIMING, 1)
             out = g4d.render(cam_of(step, v), pc, Pipe, bg)      # same binding in warm-up and timed steps
+            if kept is not None:
+                kept.append(out)
         ws.set_option(lib.OPT_STAGE_TIMING, 0)
         return out
+
+    # --dump-outputs: every step (warm-up included, so that the allocator is warm) keeps its views' outputs until the next
+    kept = [] if args.dump_outputs else None
 
     ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(K)]
     sampler = ClockSampler(local)
@@ -292,24 +300,28 @@ def run_ours(args):
     with torch.no_grad():
         for i in range(Wm):
             flush.fill_(i & 0xFF)
-            out = resident_step(i)
+            out = resident_step(i, kept)
         gc.collect(); gc.disable()     # a host hiccup shows up 1:1 in a ~1 ms view
         barrier()
         # ranks leave the collective barrier at different times and an idle B200 drops its clocks within milliseconds:
         # one more untimed step, then the synchronize that brackets the timed region
-        out = resident_step(Wm)
+        out = resident_step(Wm, kept)
         torch.cuda.synchronize(dev)
         sampler.mark()
         t_wall0 = time.perf_counter()
         for i in range(K):
             flush.fill_(i & 0xFF)
             ev[i][0].record()
-            out = resident_step(Wm + i)
+            out = resident_step(Wm + i, kept)
             ev[i][1].record()
         barrier()
         t_wall = time.perf_counter() - t_wall0
         gc.enable()
     step_ms = [a.elapsed_time(b) for a, b in ev]
+    if kept is not None:
+        if rank == 0:
+            dump_outputs(args.dump_outputs, kept)
+        kept = None
     # the stage events of the last view of the last timed step (same context: no-grad renders release it at once)
     in_region_stage_ms = ws._free_contexts[-1].stage_times() if ws._free_contexts else {}
     total_ms = _max_over_ranks(dist, dev, sum(step_ms))
@@ -387,7 +399,7 @@ def run_ours(args):
     # ------------------------------------------------------------------ training step (B=2 views, fwd+bwd, all-reduce, Adam)
     train = None
     if not args.no_train:
-        train = run_train_steps(g4d, synth, lib, w, scene, mod, dev, dist, world, rank, max(3, min(K, 10)), 5, flush)
+        train = run_train_steps(g4d, synth, lib, w, scene, mod, dev, dist, world, rank, K, 5, flush)
     clocks = sampler.stop() if rank == 0 else None     # sampled from the start of the timed region to the end of the train steps
 
     eager = None
@@ -490,6 +502,29 @@ def run_ours(args):
         print(json.dumps(line))
     if dist is not None:
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 60 * 10 ** 6      # data of the --dump-outputs files; with their headers they stay under 64 MB
+
+
+def dump_outputs(path, outs):
+    """Writes what render() returned for each view of the last timed step as PATH/<key>.npy, float32, views stacked on the
+    first axis.  When the step's outputs exceed DUMP_BYTES, every key keeps the same fraction of each view's elements, at
+    positions drawn with a fixed seed: (views, sampled elements), the same positions in every view and in every run."""
+    os.makedirs(path, exist_ok=True)
+    keys = sorted(outs[0])
+    per_view = {k: outs[0][k].numel() for k in keys}
+    frac = min(1.0, DUMP_BYTES / (4.0 * len(outs) * sum(per_view.values())))
+    for k in keys:
+        n = per_view[k]
+        m = max(1, int(n * frac))
+        if m < n:
+            idx = np.sort(np.random.default_rng(0).choice(n, m, replace=False))
+            idx = torch.from_numpy(idx).to(outs[0][k].device)
+            arr = torch.stack([o[k].reshape(-1)[idx] for o in outs])
+        else:
+            arr = torch.stack([o[k] for o in outs])
+        np.save(os.path.join(path, k + ".npy"), arr.float().cpu().numpy())
 
 
 LAUNCH_LIST = (["pack_camera", "collapse_time_rows", "deform_features", "deform_f16_kernel", "bin_sort (cooperative)",
@@ -716,10 +751,9 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps = min(args.steps, 8)          # one step = one full view (~1-2 s of CPU work): bounded sample
-    line = cpu_reference_arm(args.workload, steps=steps, warmup=min(args.warmup, 2))
+    # one step = one full view (~1-2 s of CPU work)
+    line = cpu_reference_arm(args.workload, steps=args.steps, warmup=min(args.warmup, 2))
     line["n_gpus"] = args.gpus
-    line["steps"] = steps
     print(json.dumps(line))
 
 
@@ -738,7 +772,13 @@ def main():
     ap.add_argument("--host-sync", dest="host_sync", action="store_true",
                     help="size the instance buffer exactly with one host read of R per forward (the reference's behaviour) "
                          "instead of the default capacity-bounded device-side binning")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="after the timed steps, write what render() returned for each view of the last timed step (rank 0's "
+                         "views) to DIR/<key>.npy as float32; a fixed, seeded sample of every output when all of them would "
+                         "exceed 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

@@ -2,8 +2,8 @@
 
 TEST / BASELINE INFRASTRUCTURE ONLY.  /root/reference does not exist on the GPU box: there the unmodified copies that
 ``oracle/make_ref.py`` put into ``oracle/_ref/`` at build() time are imported instead; callers must check
-``reference_available()`` first.  Used by ``oracle/make_golden_deform.py`` (golden vectors), by the
-``not gpu`` tests that pin ``oracle/deform_ref.py``, and by ``bench.py --impl reference`` when present.
+``reference_available()`` first.  Used by the ``oracle/make_golden_*.py`` scripts (the golden vectors the tests
+compare against) and by ``bench.py --impl reference`` when present.
 
 Two shims make the module importable without the reference's heavy dependencies (SURVEY §8c):
   * an empty package object ``scene`` whose ``__path__`` points at /root/reference/scene, so

@@ -1,5 +1,6 @@
 """N3 (SURVEY 8f): ply / deformation.pth round trips in the reference's formats, on CPU (no kernels involved)."""
 import importlib
+import json
 import os
 
 import numpy as np
@@ -9,8 +10,7 @@ import torch
 ck = importlib.import_module("4dgaussians_b200.checkpoint")
 synth = importlib.import_module("4dgaussians_b200.synth")
 g4d = importlib.import_module("4dgaussians_b200")
-from oracle import deform_ref as dr
-from oracle.ref_loader import load_reference_deform_network, reference_available
+REF_LAYOUT = os.path.join(os.path.dirname(__file__), "golden", "ref_state_dicts.json")
 
 
 def test_ply_round_trip_and_layout(tmp_path):
@@ -56,17 +56,20 @@ def test_deformation_pth_round_trip_both_ways(tmp_path):
     for (k, a), (k2, b) in zip(mod.state_dict().items(), other.state_dict().items()):
         assert k == k2 and torch.equal(a, b), k
     assert other.deformation_net.grid.grids[0][0].is_contiguous(memory_format=torch.channels_last) or True
-    if reference_available():     # a file written here loads in the reference's own module, and vice versa
-        cfg = dr.CONFIGS["dynerf"]
-        ref = load_reference_deform_network(cfg)
-        ref.load_state_dict(torch.load(os.path.join(d, "deformation.pth")))
-        d2 = str(tmp_path / "ref_iter")
-        os.makedirs(d2)
-        torch.save(ref.state_dict(), os.path.join(d2, "deformation.pth"))
-        third = g4d.deform_network(synth.hidden_args("dynerf"))
-        ck.load_model(d2, third, 5, device="cpu")
-        for (k, a), (_, b) in zip(mod.state_dict().items(), third.state_dict().items()):
-            assert torch.equal(a, b), k
+    # a file written here loads in the reference's own module (its strict load_state_dict wants exactly its keys and shapes,
+    # tests/golden/ref_state_dicts.json), and vice versa: the file that module writes after loading ours (its own contiguous
+    # tensors, in its key order) loads here
+    with open(REF_LAYOUT) as f:
+        layout = json.load(f)["dynerf"]["state_dict"]
+    sd = torch.load(os.path.join(d, "deformation.pth"))
+    assert [(k, list(v.shape), str(v.dtype)) for k, v in sd.items()] == [tuple(e) for e in layout]
+    d2 = str(tmp_path / "ref_iter")
+    os.makedirs(d2)
+    torch.save({k: sd[k].clone().contiguous() for k, _, _ in layout}, os.path.join(d2, "deformation.pth"))
+    third = g4d.deform_network(synth.hidden_args("dynerf"))
+    ck.load_model(d2, third, 5, device="cpu")
+    for (k, a), (_, b) in zip(mod.state_dict().items(), third.state_dict().items()):
+        assert torch.equal(a, b), k
 
 
 def test_iteration_dir_names():

@@ -1,14 +1,17 @@
 """Host-side logic of the drop-in modules that needs no GPU: state_dict compatibility with the reference module,
 parameter grouping, time-scalar quirks, settings tuple, oracle-side composition helpers used by the GPU tests."""
 import importlib
+import json
+import os
 
 import numpy as np
 import pytest
 import torch
 
-from oracle import deform_ref as dr
-from oracle.ref_loader import load_reference_deform_network, reference_available
 from util_scene import g4d, make_module, oracle_params_from_module, oracle_render, synth
+
+# the reference deform_network's state_dict layout and parameter groups (oracle/make_golden_reference.py)
+REF_LAYOUT = os.path.join(os.path.dirname(__file__), "golden", "ref_state_dicts.json")
 
 
 def test_state_dict_keys_shapes_and_layout():
@@ -32,19 +35,24 @@ def test_state_dict_keys_shapes_and_layout():
     assert g4d.deform_network(synth.hidden_args("dnerf")).head_mask() == 7
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not present")
 @pytest.mark.parametrize("name", ["dnerf", "hypernerf", "dynerf"])
 def test_state_dict_round_trips_with_reference_module(name):
+    with open(REF_LAYOUT) as f:
+        ref = json.load(f)[name]
     mine = g4d.deform_network(synth.hidden_args(name))
-    ref = load_reference_deform_network(dr.CONFIGS[name])
-    assert list(ref.state_dict().keys()) == list(mine.state_dict().keys())
-    for k, v in ref.state_dict().items():
-        assert mine.state_dict()[k].shape == v.shape, k
-    ref.load_state_dict(mine.state_dict())
-    mine.load_state_dict(ref.state_dict())
+    sd = mine.state_dict()
+    # same keys in the same order, same shapes and dtypes: the reference's strict load_state_dict accepts ours
+    assert list(sd.keys()) == [k for k, _, _ in ref["state_dict"]]
+    for k, shape, dtype in ref["state_dict"]:
+        assert list(sd[k].shape) == shape and str(sd[k].dtype) == dtype, k
+    # and ours loads what the reference's state_dict() holds: plain contiguous tensors of its layout
+    g = torch.Generator().manual_seed(0)
+    theirs = {k: torch.rand(shape, generator=g).to(getattr(torch, dtype.split(".")[1])) for k, shape, dtype in ref["state_dict"]}
+    mine.load_state_dict(theirs)
+    assert all(torch.equal(v, theirs[k]) for k, v in mine.state_dict().items())
     assert mine.deformation_net.grid.grids[0][0].is_contiguous(memory_format=torch.channels_last)
-    assert [p.shape for p in mine.get_mlp_parameters()] == [p.shape for p in ref.get_mlp_parameters()]
-    assert [p.shape for p in mine.get_grid_parameters()] == [p.shape for p in ref.get_grid_parameters()]
+    assert [list(p.shape) for p in mine.get_mlp_parameters()] == ref["mlp_parameters"]
+    assert [list(p.shape) for p in mine.get_grid_parameters()] == ref["grid_parameters"]
 
 
 def test_flat_parameter_cache_follows_the_module():
