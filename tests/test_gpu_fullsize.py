@@ -1,6 +1,7 @@
 """Full-size GPU parity: BASELINE.json configs C1 (70k, 800x800, dnerf net -> FFMA kernels), C2 (200k, 536x960, hypernerf
-net, L=3) and C3 (300k, 1352x1014, dynerf net, 5 heads) against the CPU oracle -- the sizes at which the persistent tile
-loops (148 CTAs x 16 tiles), the 85 x 64 tile grid, ~3 M tile instances and the chunked counting placement actually run.
+net, L=3), C3 (300k, 1352x1014, dynerf net, 5 heads) and C4 (2M, 1920x1080, dynerf net, ~28 M tile instances) against the
+CPU oracle -- the sizes at which the persistent tile loops (148 CTAs x 16 tiles), the 85 x 64 tile grid, millions of tile
+instances and the chunked counting placement actually run.  The backward at these sizes: test_gpu_backward_fullsize.py.
 
 Structure of the proof for the fused path (SURVEY 7 "bit-exact ... given identical post-deformation inputs"):
   (i)   the deformed + activated tensors the fused kernel produced are within fp32 rounding of the oracle's deformation;
@@ -21,7 +22,8 @@ import torch
 
 from oracle import deform_ref as dr
 from oracle import raster_ref as rr
-from util_scene import cam_tuple, g4d, make_module, oracle_params_from_module, oracle_render, raster_inputs, rel_err, synth
+from util_scene import (_assert_index_data_bit_exact, cam_tuple, g4d, make_module, oracle_params_from_module, oracle_render,
+                        raster_inputs, rel_err, synth)
 
 pytestmark = pytest.mark.gpu
 IMG_TOL = 1e-4
@@ -54,32 +56,6 @@ def _settings(cam, bg, sh_degree=3, dev="cuda"):
         campos=cam.camera_center.to(dev), prefiltered=False, debug=False)
 
 
-def _assert_index_data_bit_exact(ctx, radii_gpu, ref, colour_exact=True):
-    pr, bn = ref["proj"], ref["bin"]
-    assert np.array_equal(radii_gpu, ref["radii"])
-    for name, want in (("depth", pr.depth), ("rect", pr.rect), ("tiles_touched", pr.tiles_touched), ("xy", pr.xy),
-                       ("conic_opacity", pr.conic_op), ("rgb", pr.rgb), ("clamped", pr.clamped)):
-        got = ctx.read(name)
-        assert got.shape == want.shape, name
-        if name in ("rgb", "clamped") and not colour_exact:
-            # the fused tensor-core kernel evaluates the SH polynomial with all 16 basis values in registers (a different
-            # association order from the standalone preprocess kernel) and also for culled Gaussians (whose colour nobody
-            # reads): colours of the VISIBLE Gaussians agree to fp32 rounding, not bit for bit
-            vis = ref["radii"] > 0
-            if name == "rgb":
-                assert float(np.abs(got[vis] - want[vis]).max()) <= 2e-6, name
-            else:
-                assert float((got[vis] != want[vis]).mean()) <= 1e-4, name
-            continue
-        assert np.array_equal(got.view(np.uint8), want.view(np.uint8)), name
-    st = ctx.stats()
-    assert st.num_rendered == bn.R and st.num_visible == int((ref["radii"] > 0).sum())
-    assert np.array_equal(ctx.read("sorted_ids"), bn.ids)
-    assert np.array_equal(ctx.read("ranges"), bn.ranges)
-    assert np.array_equal(ctx.read("sorted_keys"), bn.keys)
-    return bn.R
-
-
 def _assert_pixel_outliers_are_threshold_flips(img_gpu, ref, W, max_outliers_frac=2e-5, max_err=6e-3):
     """Pixels where the GPU image is off by more than 1e-4 must be pixels where a DISCRETE decision of the compositing loop
     (A.3) sits within fp32 rounding of its threshold for one of the pixel's instances: alpha >= 1/255 (a skipped / kept
@@ -107,7 +83,7 @@ def _assert_pixel_outliers_are_threshold_flips(img_gpu, ref, W, max_outliers_fra
     return len(ys), float(err.max())
 
 
-@pytest.mark.parametrize("wl", ["C1", "C2", "C3"])
+@pytest.mark.parametrize("wl", ["C1", "C2", "C3", "C4"])
 @pytest.mark.parametrize("sync_mode", [1, 0])
 def test_full_size_rasterizer_forward_vs_oracle(wl, sync_mode):
     """Drop-in GaussianRasterizer at BASELINE sizes: every index array bit-exact, image L-inf <= 1e-4.  sync_mode 0 = the
@@ -174,7 +150,7 @@ def test_full_size_rasterizer_backward_C3_vs_oracle():
         assert e <= GRAD_TOL, (nm, e)
 
 
-@pytest.mark.parametrize("wl", ["C1", "C2", "C3"])
+@pytest.mark.parametrize("wl", ["C1", "C2", "C3", "C4"])
 def test_full_size_fused_forward_vs_oracle(wl):
     w = synth.WORKLOADS[wl]
     scene = synth.make_scene(w["n"], seed=0, scale_mean=w["scale_mean"])
